@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — the hot path of BASELINE.json on B200: rows/s and fraction of HBM roofline, filter AND aggregate.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--rows R]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--rows R] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Headline workload (BASELINE.json configs[1], "C2"): SELECT a FROM t WHERE a > 0.5 over 1e8 synthetic Float64
@@ -18,7 +18,8 @@ next to it (`roofline_c4`, `e2e_c4`, `cpu_baseline_c4`); C3 and C5 are in `extra
                 by row-range chunk inside the library
   roofline      algorithmic bytes of the dominant kernel (8*N read + 8*N_sel written) / its average duration
                 measured with CUDA events recorded around the launch on the launching stream
-  sustained     the same resident step repeated back to back for >= 0.5 s (the K timed steps of C2 last a few ms)
+  sustained     with --sustained only: the same resident step repeated back to back for >= 0.5 s (the K timed
+                steps of C2 last a few ms)
   roofline_c4   the same for k_hash_agg (16*N bytes read), e2e_c4 through dfgpu_aggregate_update_host
   extra         C3 (fused expr+filter) and C5 (1e6 keys, MIN/MAX/SUM, 1.25e8 rows per GPU = 1e9 rows on 8 GPUs;
                 with N>1 C4 and C5 include the NCCL partial-aggregate merge), same timing rules
@@ -29,6 +30,16 @@ next to it (`roofline_c4`, `e2e_c4`, `cpu_baseline_c4`); C3 and C5 are in `extra
 
 --impl reference times that CPU restatement alone (the reference is Rust; no toolchain here) on the SAME
 config: one full 1e8-row C2 batch per step.
+
+Every timed loop (value, e2e, C3, C4, e2e_c4, C5) runs exactly K = --steps steps after its warm-ups.
+
+--dump-outputs DIR writes, on rank 0, what the last timed step returned to its caller, as DIR/<name>.npy:
+  c2_a                        the C2 result column (Float64); above 4 Mi rows, the rows at 4 Mi positions drawn
+                              once with numpy's default_rng(0) and kept in ascending order (32 MB)
+  c4_key_hi, c4_key_lo        the C4 GROUP BY keys (Int64) as their signed high and unsigned low 32 bits, Float64
+  c4_sum, c4_count            SUM(v) and COUNT(v) of C4 (Float64), all rows sorted by key (the engine's row order
+                              is that of its hash table and may differ from run to run)
+The inputs are seeded, so two runs with the same arguments see the same rows.
 """
 import argparse
 import json
@@ -40,11 +51,14 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True  # a benchmark run leaves the source tree as it found it (no __pycache__)
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
 METRIC = "rows/s filter+agg over 1e8-row Arrow batch (C2: SELECT a FROM t WHERE a>0.5, Float64)"
 SUM_RTOL = 1e-9
+DUMP_SAMPLE_ROWS = 1 << 22  # --dump-outputs: at most 4 Mi rows (32 MB of Float64) of the C2 result column
+DUMP_MAX_BYTES = 64 << 20
 
 
 def c2_config(n):
@@ -151,7 +165,7 @@ class ClockSampler:
             reasons = sorted({nm for _, rs, _ in self.samples for nm, b in bits.items() if rs & b})
             sm = [x[0] for x in self.samples]
             return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": mx, "power_w_max": max([x[2] for x in self.samples], default=None),
-                    "samples": len(sm), "reasons": reasons, "source": "nvml, ~2 ms period, warm-up + timed steps + sustained loop"}
+                    "samples": len(sm), "reasons": reasons, "source": "nvml, ~2 ms period, warm-up + timed steps (+ sustained loop)"}
         if not self.proc:
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["nvidia-smi unavailable"]}
         time.sleep(0.15)
@@ -226,8 +240,9 @@ def allreduce_np(torch, arr, op):
     return t.cpu().numpy()
 
 
-def time_steps(ctx, torch, fn, steps, warmup):
-    """W untimed warm-ups, then exactly K steps between barrier+sync, device events, max over ranks."""
+def time_steps(ctx, torch, fn, steps, warmup, last=None):
+    """W untimed warm-ups, then exactly K steps between barrier+sync, device events, max over ranks.
+    `last`, if given, is the K-th step: the same work as `fn`, but it keeps its result for the caller."""
     for _ in range(warmup):
         fn()
     ctx.sync()
@@ -235,14 +250,32 @@ def time_steps(ctx, torch, fn, steps, warmup):
     ctx.profile_enable(True)
     l0 = ctx.kernel_launches()
     ctx.timer_start()
-    for _ in range(steps):
-        fn()
+    for i in range(steps):
+        (last if last is not None and i == steps - 1 else fn)()
     ms = ctx.timer_stop()
     ctx.sync()
     barrier(torch)
     kms, kn = ctx.profile_get()
     ctx.profile_enable(False)
     return max_over_ranks(torch, ms), kms, kn, ctx.kernel_launches() - l0
+
+
+def dump_sample(x):
+    """`x` whole if it has at most DUMP_SAMPLE_ROWS rows, else its rows at DUMP_SAMPLE_ROWS positions drawn with
+    default_rng(0), ascending: the same positions for the same length."""
+    if len(x) <= DUMP_SAMPLE_ROWS:
+        return x
+    return x[np.sort(np.random.default_rng(0).choice(len(x), DUMP_SAMPLE_ROWS, replace=False))]
+
+
+def write_outputs(d, arrays):
+    """--dump-outputs: one DIR/<name>.npy per array, Float64 only, DUMP_MAX_BYTES in all."""
+    assert all(a.dtype == np.float64 for a in arrays.values())
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_MAX_BYTES, "outputs to dump: %d bytes" % total
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), np.ascontiguousarray(a))
 
 
 def check_groupby(torch, got, k_raw, v, nkeys, want, what):
@@ -289,7 +322,8 @@ def run_ours(args):
     ctx = engine.GpuContext(local)
     peak, peak_src = hbm_peak()
     n = args.rows
-    steps, warmup = (args.steps or 2000), max(3, args.warmup)
+    steps, warmup = args.steps, max(3, args.warmup)
+    dumps = {}  # --dump-outputs: name -> array
 
     # ---- C2 (headline) -----------------------------------------------------------------------
     pin_in = engine.PinnedBuffer((n,), np.float64)
@@ -299,10 +333,13 @@ def run_ours(args):
     batch = ctx.upload([a])
     state = {}
 
-    def step_resident():
+    def step_resident(keep=False):
         r = ctx.filter_project(batch, pred, proj)
         state["nrows"] = r.nrows
-        r.free()
+        if keep:
+            state["r2"] = r
+        else:
+            r.free()
 
     def step_e2e():
         # the call a user of the engine makes for a host-resident batch: host buffers in, host buffers
@@ -314,18 +351,23 @@ def run_ours(args):
 
     sampler = ClockSampler(local)
     sampler.start()
-    ms, kms, kn, launches = time_steps(ctx, torch, step_resident, steps, warmup)
+    ms, kms, kn, launches = time_steps(ctx, torch, step_resident, steps, warmup, last=lambda: step_resident(keep=True))
     assert state["nrows"] == n_sel, "GPU row count %d != expected %d" % (state["nrows"], n_sel)
-    # sustained: the same step back to back for >= 0.5 s (same kernel, clocks sampled throughout)
-    sus_steps = steps if args.no_sustained else max(steps, int(np.ceil(600.0 / max(ms / steps, 1e-3))))
-    sms, skms, skn, _ = time_steps(ctx, torch, step_resident, sus_steps, 0)
+    r2 = state.pop("r2")
+    if args.dump_outputs:
+        dumps["c2_a"] = dump_sample(r2.columns()[0])
+    r2.free()
+    if args.sustained:
+        # the same step back to back for >= 0.5 s (same kernel, clocks sampled throughout)
+        sus_steps = max(steps, int(np.ceil(600.0 / max(ms / steps, 1e-3))))
+        sms, skms, skn, _ = time_steps(ctx, torch, step_resident, sus_steps, 0)
     clocks = sampler.stop()
     total_rows = sum_over_ranks(torch, float(n))
     value = total_rows * steps / (ms / 1e3)
     kernel_ms = kms / steps  # device time of the dominant kernel per step (1 launch per step here)
     alg_bytes = 8.0 * n + 8.0 * n_sel
     achieved = alg_bytes / (kernel_ms / 1e3) / 1e9
-    e2e_steps = max(3, min(steps, 10))
+    e2e_steps = steps
     ems, _, _, _ = time_steps(ctx, torch, step_e2e, e2e_steps, 3)
     assert state["nrows"] == n_sel and np.array_equal(state["e2e_out"], a[a > 0.5][:1000])
     e2e_value = total_rows * e2e_steps / (ems / 1e3)
@@ -344,13 +386,14 @@ def run_ours(args):
         "roofline": {"bound": "hbm", "achieved": achieved, "peak": peak, "unit": "GB/s", "frac": achieved / peak,
                      "traffic": ncu_traffic("k_filter_project:c2") if n == 100_000_000 else None, "kernel": "k_filter_project_tma", "kernel_ms": kernel_ms,
                      "algorithmic_bytes": alg_bytes, "peak_source": peak_src},
-        "sustained": {"steps": sus_steps, "seconds": sms / 1e3, "ms_per_step": sms / sus_steps, "kernel_ms": skms / sus_steps,
-                      "value": total_rows * sus_steps / (sms / 1e3), "roofline_frac": alg_bytes / (skms / sus_steps / 1e3) / 1e9 / peak},
     }
+    if args.sustained:
+        out["sustained"] = {"steps": sus_steps, "seconds": sms / 1e3, "ms_per_step": sms / sus_steps, "kernel_ms": skms / sus_steps,
+                            "value": total_rows * sus_steps / (sms / 1e3), "roofline_frac": alg_bytes / (skms / sus_steps / 1e3) / 1e9 / peak}
 
     # ---- C3 (extra) ---------------------------------------------------------------------------------
     extra = {}
-    xs = max(3, min(steps, 10))
+    xs = steps
     try:
         arrays3, pred3, proj3 = workloads.c3(n, seed=142 + 10 * rank)
         b3 = ctx.upload(arrays3[:2])  # c, d are never referenced: not uploaded (the host layer prunes them the same way)
@@ -388,23 +431,31 @@ def run_ours(args):
     arrays4 = [pin_k.array, pin_v.array]
     b4 = ctx.upload(arrays4)
 
-    def step4():
+    def step4(keep=False):
         r = ctx.aggregate(b4, keys4, aggs4)
         state["g4"] = r.nrows
-        if "keep4" in state:
-            state["cols4"] = r.columns()
-        r.free()
+        if keep:
+            state["r4"] = r
+        else:
+            r.free()
 
     def step4_e2e():
         r = ctx.aggregate_host(arrays4, keys4, aggs4)
         state["g4e"] = r.nrows
         state["cols4e"] = r.columns()  # D2H of the (small) result is part of the step
         r.free()
-    ms4, kms4, kn4, _ = time_steps(ctx, torch, step4, xs, 3)
-    state["keep4"] = True
-    step4()
-    del state["keep4"]
-    chk4 = check_groupby(torch, state["cols4"], kraw4, arrays4[1], 100_000, ["sum", "count"], "C4")
+    ms4, kms4, kn4, _ = time_steps(ctx, torch, step4, xs, 3, last=lambda: step4(keep=True))
+    r4 = state.pop("r4")
+    cols4 = r4.columns()
+    r4.free()
+    chk4 = check_groupby(torch, cols4, kraw4, arrays4[1], 100_000, ["sum", "count"], "C4")
+    if args.dump_outputs:
+        o = np.argsort(cols4[0], kind="stable")
+        k = cols4[0][o]
+        dumps["c4_key_hi"] = (k >> 32).astype(np.float64)
+        dumps["c4_key_lo"] = (k & 0xFFFFFFFF).astype(np.float64)
+        dumps["c4_sum"] = cols4[1][o].astype(np.float64)
+        dumps["c4_count"] = cols4[2][o].astype(np.float64)
     k4 = kms4 / xs  # scan kernel time per step (a first batch runs two launches: 1 Mi-row sampled prefix + the rest)
     bytes4 = 16.0 * n
     out["roofline_c4"] = {"bound": "hbm", "achieved": bytes4 / (k4 / 1e3) / 1e9, "peak": peak, "unit": "GB/s",
@@ -428,16 +479,18 @@ def run_ours(args):
         arrays5, keys5, aggs5, kraw5 = workloads.c5(n5, seed=46 + 10 * rank)
         b5 = ctx.upload(arrays5)
 
-        def step5():
+        def step5(keep=False):
             r = ctx.aggregate(b5, keys5, aggs5)
             state["g5"] = r.nrows
-            if "keep5" in state:
-                state["cols5"] = r.columns()
-            r.free()
-        ms5, kms5, kn5, _ = time_steps(ctx, torch, step5, xs, 3)
-        state["keep5"] = True
-        step5()
-        chk5 = check_groupby(torch, state["cols5"], kraw5, arrays5[1], 1_000_000, ["min", "max", "sum"], "C5")
+            if keep:
+                state["r5"] = r
+            else:
+                r.free()
+        ms5, kms5, kn5, _ = time_steps(ctx, torch, step5, xs, 3, last=lambda: step5(keep=True))
+        r5 = state.pop("r5")
+        cols5 = r5.columns()
+        r5.free()
+        chk5 = check_groupby(torch, cols5, kraw5, arrays5[1], 1_000_000, ["min", "max", "sum"], "C5")
         k5 = kms5 / xs
         bytes5 = 16.0 * n5
         total5 = sum_over_ranks(torch, float(n5))
@@ -461,6 +514,8 @@ def run_ours(args):
         out["cpu_baseline_c4"] = cpu_baseline_c4(arrays4, keys4, aggs4)
     ctx.close()
     if rank == 0:
+        if args.dump_outputs:
+            write_outputs(args.dump_outputs, dumps)
         print(json.dumps(out))
     if torch is not None:
         import torch.distributed as dist
@@ -511,7 +566,7 @@ def run_reference(args):
     from datafusion_archive_b200 import workloads
     n = args.rows
     arrays, pred, proj = workloads.c2(n, seed=42)
-    steps, warmup = (args.steps or 5), max(3, args.warmup)
+    steps, warmup = args.steps, max(3, args.warmup)
     state = {}
     for _ in range(warmup):
         state["out"] = O.filter_project(arrays, pred, proj)
@@ -539,14 +594,19 @@ def run_reference(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=None, help="timed steps (default: 2000 resident steps = ~0.6 s; reference arm: 5)")
+    ap.add_argument("--steps", type=int, default=None, help="timed steps of every timed loop (default: 20; reference arm: 5)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--rows", type=int, default=100_000_000, help="rows per GPU")
     ap.add_argument("--rows5", type=int, default=0, help="rows per GPU of the C5 extra (default 1.25 x --rows)")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline legs")
-    ap.add_argument("--no-sustained", action="store_true", help="keep the sustained loop as short as the timed steps (for ncu launch lists)")
+    ap.add_argument("--sustained", action="store_true", help="also repeat the C2 step back to back for >= 0.5 s (reported as `sustained`)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's C2 and C4 results to DIR/<name>.npy (Float64)")
     args = ap.parse_args()
+    if args.steps is None:
+        args.steps = 5 if args.impl == "reference" else 20
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -9,7 +9,7 @@ timeout 400 python -m pytest tests -m gpu -x -q 2>&1 | tail -3 | tee $out/${tag}
 timeout 60 python -c "import __graft_entry__ as g; g.smoke(); print('SMOKE_OK')" 2>&1 | tail -2 | tee $out/${tag}_smoke.txt
 timeout 400 python bench.py --steps 20 --warmup 5 2> $out/${tag}_bench.err | tail -1 > $out/${tag}_bench.json
 timeout 300 python bench.py --impl reference --steps 20 --warmup 5 2>> $out/${tag}_bench.err | tail -1 > $out/${tag}_bench_reference.json
-timeout 300 ncu --metrics gpu__time_duration.sum --clock-control none -c 2000 --csv --log-file $out/${tag}_launches.csv python bench.py --steps 2 --warmup 3 --no-cpu --no-sustained > /dev/null 2>&1
+timeout 300 ncu --metrics gpu__time_duration.sum --clock-control none -c 2000 --csv --log-file $out/${tag}_launches.csv python bench.py --steps 2 --warmup 3 --no-cpu > /dev/null 2>&1
 python profiles/launch_shares.py $out/${tag}_launches.csv > $out/${tag}_launch_shares.txt 2>&1
 for w in c2 c3 c4 c5 reduce; do
   k=k_filter_project; [ $w = c4 ] && k=k_hash_agg; [ $w = c5 ] && k=k_hash_agg; [ $w = reduce ] && k=k_reduce

@@ -45,7 +45,7 @@ def test_gloo_world2_partition_and_merge():
 def test_nccl_world2_partial_aggregate_merge():
     from datafusion_archive_b200 import engine
     if engine.device_count() < 2:
-        pytest.skip("needs 2 GPUs (run under gpurun --gpus 2)")
+        pytest.skip("needs 2 GPUs")
     p = launch("nccl", 2, 29632)
     assert p.returncode == 0, p.stdout[-2000:] + p.stderr[-4000:]
     assert "MP_OK mode=nccl world=2" in p.stdout
